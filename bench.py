@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (own arm; torchrun for N > 1)
   python bench.py --impl reference --gpus N --steps K ...  (upstream's CPU path, rank 0 only)
+  python bench.py ... --dump-outputs DIR                   (also save what the last timed step computed)
 
 Workload (BASELINE.json configs[2]): CImageResizer<fpclass_float8_avx-equiv> 7680x4320 ->
 3840x2160, 4-channel float.  A "step" resizes one such frame per GPU.  For N > 1 the N frames
@@ -35,6 +36,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -582,6 +584,8 @@ def run_own(args):
     total_ms = timed(step, args.steps, args.warmup)
     t1 = time.time()
     clocks = sampler.stop(t0, t1) if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, d_dst, "output" if N == 1 else "output_rank%d" % rank, N)
     launches_per_step = lib.avirb200_plan_last_launches(pl.plan)
     ms_per_step = total_ms / args.steps
     value = SRC_W * SRC_H * N / (ms_per_step * 1e-3) / 1e6
@@ -821,6 +825,21 @@ def run_own(args):
     pl.close()
 
 
+DUMP_ROWS = 512  # rows of the 3840-wide RGBA float destination: 31.5 MB over all ranks
+
+
+def dump_outputs(d, d_dst, name, n_ranks):
+    """Saves what the last timed step left in d_dst (the caller's destination image): a fixed,
+    seeded sample of whole rows, DIR/<name>.npy (float32, rows x DST_W x CH), and the row numbers
+    within the band, DIR/<name>_rows.npy (float64)."""
+    rows = np.sort(np.random.default_rng(0).choice(d_dst.shape[0], min(d_dst.shape[0], DUMP_ROWS // n_ranks),
+                                                   replace=False))
+    import torch
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, name + ".npy"), d_dst.index_select(0, torch.as_tensor(rows, device=d_dst.device)).cpu().numpy())
+    np.save(os.path.join(d, name + "_rows.npy"), rows.astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -832,6 +851,8 @@ def main():
     ap.add_argument("--halo-mode", type=int, default=None, choices=[0, 1, 2, 3],
                     help="sharded runs: AVIRB200_OPT_OVERLAP_HALO (default: the library's)")
     ap.add_argument("--no-extras", action="store_true", help="headline only (no secondary configs / LANCIR / variants)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/*.npy (a seeded sample of its rows)")
     args = ap.parse_args()
     Plan.halo_mode = args.halo_mode
     args.warmup = max(args.warmup, 3) if args.impl == "own" else args.warmup

@@ -174,6 +174,76 @@ def count_mismatch(a, b):
     return int((a != b).sum())
 
 
+# ---- upstream's outputs, stored as digests -------------------------------------------------------
+# Every comparison with upstream goes through upstream(): it returns the digest of the output upstream
+# (oracle/_ref) produced for a key naming the call and its input, read from tests/golden/upstream.json,
+# so the suite needs neither the reference sources nor oracle/_ref.  With AVIRB200_RECORD_UPSTREAM=<file>
+# set (and oracle/_ref built) it runs upstream instead and merges every key it computed into <file>;
+# tests/golden/make_golden.py describes the regeneration.
+
+UPSTREAM_JSON = os.path.join(GOLDEN, "upstream.json")
+_upstream = None
+_recorded = {}
+
+
+def digest(a):
+    """Digest of an array's shape, type and bits (+0.0 for -0.0 in double arrays: count_mismatch
+    compares those by value)."""
+    import hashlib
+    a = np.ascontiguousarray(a)
+    if a.dtype == np.float64:
+        a = a + 0.0
+    h = hashlib.sha256(("%s%s" % (a.dtype.str, a.shape)).encode())
+    h.update(a.view(np.uint8).reshape(-1))
+    return h.hexdigest()[:32]
+
+
+def avir_key(case, src):
+    return case_id(case) + "/" + digest(src)[:16]
+
+
+def lancir_key(src, nw, nh, to, kw):
+    sh, sw, ch = src.shape
+    s = "lancir-%dx%d-%dx%d-c%d-%s-%s" % (sw, sh, nw, nh, ch, src.dtype.name, np.dtype(to).name)
+    for k_, v_ in sorted(kw.items()):
+        s += "-%s%s" % (k_, v_)
+    return s + "/" + digest(src)[:16]
+
+
+def _flush_recorded():
+    import json
+    path = os.environ["AVIRB200_RECORD_UPSTREAM"]
+    have = json.load(open(path)) if os.path.exists(path) else {}
+    have.update(_recorded)
+    with open(path, "w") as f:
+        json.dump(have, f, indent=0, sort_keys=True)
+        f.write("\n")
+
+
+def upstream(key, compute):
+    """The stored value for `key`; `compute()` runs upstream for it (record mode only) and returns
+    an array (stored as its digest) or a JSON value."""
+    global _upstream
+    if os.environ.get("AVIRB200_RECORD_UPSTREAM"):
+        assert o.have_ref(), "recording upstream's outputs needs oracle/_ref"
+        if not _recorded:
+            import atexit
+            atexit.register(_flush_recorded)
+        v = compute()
+        _recorded[key] = digest(v) if isinstance(v, np.ndarray) else v
+        return _recorded[key]
+    if _upstream is None:
+        import json
+        _upstream = json.load(open(UPSTREAM_JSON))
+    assert key in _upstream, "no stored upstream output for %s (tests/golden/make_golden.py)" % key
+    return _upstream[key]
+
+
+def matches_upstream(case, src, got):
+    """True when `got` has the bits upstream produced for this AVIR case and input."""
+    return digest(got) == upstream(avir_key(case, src), lambda: ref_output(case, src))
+
+
 def case_id(case):
     fp, sw, sh, nw, nh, ch, ti, to, rb, kw = case
     s = "%s-%dx%d-%dx%d-c%d-%s-%s-b%d" % (("def", "f4", "dil", "defE", "f4E", "dilE")[fp], sw, sh, nw, nh, ch,

@@ -6,6 +6,12 @@ Run in the build container (where /root/reference exists):
 Each avir_*.npz holds: case tuple, seeded input image, upstream's output image.
 Each lancir_*.npz holds: geometry, input, upstream CLancIR output.
 Fixtures are small (<= ~100 KB each) so they can live in git.
+
+upstream.json holds, for every other comparison of the suite and smoke() with upstream, the digest of
+upstream's output (cases.digest), keyed by the call and the digest of its input (cases.upstream).  It
+is recorded by running them with oracle/_ref built, on a machine with a B200 for the GPU tests:
+    rm tests/golden/upstream.json; export AVIRB200_RECORD_UPSTREAM=$PWD/tests/golden/upstream.json
+    python -m pytest tests; python -c "import __graft_entry__ as g; g.smoke()"
 """
 import os
 import sys

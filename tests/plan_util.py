@@ -62,69 +62,67 @@ def _bits(a):
     return np.ascontiguousarray(a, dtype=np.float32).view(np.uint32)
 
 
-def compare_axis(mine, refsteps):
-    """Returns a list of mismatch descriptions between the host plan of one axis and the
-    step list recorded from the upstream run."""
-    bad = []
+def expected_axis(refsteps):
+    """What the host plan of one axis must hold, from the step list recorded from the upstream run:
+    one dict per host step, scalars as ints and arrays as float32 bits / int32."""
+    out = []
     # fold upstream's filterless upsample step into the following resize step
-    folded = []
     pend = None
-    for s in refsteps:
-        if s["kind"] == 1 and s["FltOrigLen"] > 0:
-            pend = s  # filterless 2X upsample: folded into the next (resize) step
+    for r in refsteps:
+        if r["kind"] == 1 and r["FltOrigLen"] > 0:
+            pend = r  # filterless 2X upsample: folded into the next (resize) step
             continue
-        s = dict(s)
-        s["up_in_len"] = pend["InLen"] if pend is not None else None
-        pend = None
-        folded.append(s)
-    if len(folded) != len(mine["steps"]):
-        return ["step count %d vs ref %d" % (len(mine["steps"]), len(folded))]
-    for i, (m, r) in enumerate(zip(mine["steps"], folded)):
-        tag = "step %d: " % i
         if r["kind"] == 1:
-            if m["kind"] != 1:
-                bad.append(tag + "kind")
-                continue
-            for a, b in (("R", "R"), ("lat", "lat"), ("in_len", "InLen"), ("out_len", "OutLen"),
-                         ("out_prefix", "OutPrefix"), ("out_suffix", "OutSuffix"),
-                         ("in_prefix", "InPrefix"), ("in_suffix", "InSuffix")):
-                if m[a] != r[b]:
-                    bad.append(tag + "%s %d vs %d" % (a, m[a], r[b]))
-            if len(m["taps"]) != len(r["Flt"]) or not np.array_equal(_bits(m["taps"]), _bits(r["Flt"])):
-                bad.append(tag + "upsample taps differ")
+            e = dict(kind=1, R=r["R"], lat=r["lat"], in_len=r["InLen"], out_len=r["OutLen"],
+                     out_prefix=r["OutPrefix"], out_suffix=r["OutSuffix"], in_prefix=r["InPrefix"],
+                     in_suffix=r["InSuffix"], taps=_bits(r["Flt"]))
         elif r["kind"] == 0:
-            if m["kind"] != 0:
-                bad.append(tag + "kind")
-                continue
-            for a, b in (("R", "R"), ("lat", "lat"), ("edge", "edge"), ("in_len", "InLen"),
-                         ("out_len", "OutLen")):
-                if m[a] != r[b]:
-                    bad.append(tag + "%s %d vs %d" % (a, m[a], r[b]))
-            if len(m["taps"]) != len(r["Flt"]) or not np.array_equal(_bits(m["taps"]), _bits(r["Flt"])):
-                bad.append(tag + "FIR taps differ")
+            e = dict(kind=0, R=r["R"], lat=r["lat"], edge=r["edge"], in_len=r["InLen"], out_len=r["OutLen"],
+                     taps=_bits(r["Flt"]))
         else:
-            if m["kind"] != 2:
-                bad.append(tag + "kind")
+            e = dict(kind=2, in_len=pend["InLen"] if pend is not None else r["InLen"],
+                     upsampled=int(pend is not None), skip_odd=int(r["kind"] == 3), out_len=r["OutLen"],
+                     ntaps=r["FL"], order=r["order"], src_pos=np.asarray(r["SrcPosInt"], np.int32),
+                     frac=_bits(r["x"]),
+                     bank_taps=np.stack([_bits(r["bank"][int(r["fti"][j])]) for j in range(r["OutLen"])]))
+        pend = None
+        out.append(e)
+    return out
+
+
+def _same(a, b):
+    """b: an array, or the digest of one (as stored in tests/golden/upstream.json)."""
+    import cases as cs
+    return cs.digest(a) == b if isinstance(b, str) else np.array_equal(a, b)
+
+
+def compare_axis(mine, expected):
+    """Returns a list of mismatch descriptions between the host plan of one axis and
+    expected_axis() of upstream's steps (or its stored form, arrays as digests)."""
+    bad = []
+    if len(expected) != len(mine["steps"]):
+        return ["step count %d vs ref %d" % (len(mine["steps"]), len(expected))]
+    for i, (m, e) in enumerate(zip(mine["steps"], expected)):
+        tag = "step %d: " % i
+        if m["kind"] != e["kind"]:
+            bad.append(tag + "kind")
+            continue
+        for a, b in e.items():
+            if a in ("taps", "frac", "src_pos", "bank_taps"):
                 continue
-            exp_in = r["up_in_len"] if r["up_in_len"] is not None else r["InLen"]
-            if m["in_len"] != exp_in:
-                bad.append(tag + "in_len %d vs %d" % (m["in_len"], exp_in))
-            if m["upsampled"] != int(r["up_in_len"] is not None):
-                bad.append(tag + "upsampled flag")
-            if m["skip_odd"] != int(r["kind"] == 3):
-                bad.append(tag + "skip_odd flag")
-            for a, b in (("out_len", "OutLen"), ("ntaps", "FL"), ("order", "order")):
-                if m[a] != r[b]:
-                    bad.append(tag + "%s %d vs %d" % (a, m[a], r[b]))
-            if not np.array_equal(m["src_pos"], r["SrcPosInt"]):
-                bad.append(tag + "src_pos differ")
-            if not np.array_equal(_bits(m["frac"]), _bits(r["x"])):
-                bad.append(tag + "frac differ")
-            stride = m["ntaps"] * (m["order"] + 1)
-            tp = m["taps"].reshape(-1, stride)
-            for j in range(m["out_len"]):
-                rt = r["bank"][int(r["fti"][j])]
-                if not np.array_equal(_bits(tp[m["phase"][j]]), _bits(rt)):
-                    bad.append(tag + "bank taps differ at output %d" % j)
-                    break
+            if m[a] != b:
+                bad.append(tag + "%s %d vs %d" % (a, m[a], b))
+        if e["kind"] != 2:
+            if not _same(_bits(m["taps"]), e["taps"]):
+                bad.append(tag + ("upsample" if e["kind"] == 1 else "FIR") + " taps differ")
+            continue
+        if not _same(np.asarray(m["src_pos"], np.int32), e["src_pos"]):
+            bad.append(tag + "src_pos differ")
+        if not _same(_bits(m["frac"]), e["frac"]):
+            bad.append(tag + "frac differ")
+        stride = m["ntaps"] * (m["order"] + 1)
+        if m["out_len"] == e["out_len"] and len(m["taps"]) % stride == 0:
+            tp = _bits(m["taps"]).reshape(-1, stride)
+            if not _same(tp[np.asarray(m["phase"][:m["out_len"]])], e["bank_taps"]):
+                bad.append(tag + "bank taps differ")
     return bad

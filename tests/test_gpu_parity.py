@@ -1,7 +1,8 @@
 """GPU parity tests proper (run with -m gpu on a B200): the product path -- C++ front-end ->
-C ABI -> sm_100a kernels -- against upstream compiled in-tree (oracle/_ref, travels prebuilt),
-the C port and the committed golden fixtures.  Bit-exact everywhere: integer output AND
-float output (0 ULP; the north-star tolerance for float is 1 ULP, the tests demand 0).
+C ABI -> sm_100a kernels -- against upstream's outputs (digests in tests/golden/upstream.json,
+recorded from upstream compiled in-tree) and the committed golden fixtures.  Bit-exact
+everywhere: integer output AND float output (0 ULP; the north-star tolerance for float is 1 ULP,
+the tests demand 0).
 """
 import ctypes as C
 import os
@@ -15,9 +16,6 @@ import oracle_ref as o
 
 pytestmark = pytest.mark.gpu
 
-needs_ref = pytest.mark.skipif(not o.have_ref(), reason="oracle/_ref not built")
-
-
 def _oracle_threads():
     """Threads for the multi-threaded upstream oracle: the cores this process may actually use
     (a container often sees every host core in os.cpu_count() but is scheduled on a few;
@@ -27,12 +25,6 @@ def _oracle_threads():
     except AttributeError:
         n = os.cpu_count() or 8
     return max(1, min(n, 16))
-
-
-def expected(case, src):
-    if o.have_ref():
-        return cs.ref_output(case, src)
-    return cs.port_output(case, src)[0]
 
 
 @pytest.fixture(params=[0, 2, 1], ids=["product", "tile", "generic"])
@@ -55,7 +47,7 @@ def test_native_library_is_what_runs():
 def test_small_cases_bit_exact(case, kernel_path):
     src = cs.make_input(case)
     got = cs.gpu_output(case, src)
-    assert cs.count_mismatch(expected(case, src), got) == 0
+    assert cs.matches_upstream(case, src, got)
 
 
 @pytest.mark.parametrize("structured", ["ramp", "impulse", "checker"])
@@ -63,7 +55,7 @@ def test_small_cases_bit_exact(case, kernel_path):
 def test_structured_inputs_bit_exact(case, structured, kernel_path):
     src = cs.make_input(case, structured=structured)
     got = cs.gpu_output(case, src)
-    assert cs.count_mismatch(expected(case, src), got) == 0
+    assert cs.matches_upstream(case, src, got)
 
 
 def test_golden_fixtures():
@@ -99,18 +91,20 @@ MEDIUM = [
 ]
 
 
-@needs_ref
+def _upstream_mt(case, src):
+    """Upstream's output digest; recording runs upstream multi-threaded (same bits)."""
+    fp, sw, sh, nw, nh, ch, ti, to, rb, kw = case
+    return cs.upstream(cs.avir_key(case, src), lambda: o.ref_resize(
+        src, nw, nh, to, fpclass=fp, resbits=rb, nthreads=_oracle_threads(), **cs.ref_kwargs(kw)))
+
+
 @pytest.mark.parametrize("case", MEDIUM, ids=cs.case_id)
 def test_medium_cases_bit_exact(case):
-    fp, sw, sh, nw, nh, ch, ti, to, rb, kw = case
     src = cs.make_input(case, seed=11)
-    ref = o.ref_resize(src, nw, nh, to, fpclass=fp, resbits=rb, nthreads=_oracle_threads(),
-                       **cs.ref_kwargs(kw))
     got = cs.gpu_output(case, src)
-    assert cs.count_mismatch(ref, got) == 0
+    assert cs.digest(got) == _upstream_mt(case, src)
 
 
-@needs_ref
 def test_generic_and_fast_kernels_agree_on_medium():
     case = MEDIUM[0]
     src = cs.make_input(case, seed=5)
@@ -142,7 +136,7 @@ def test_deselected_streaming_chains_bit_exact(case):
         got = cs.gpu_output(case, src)
     finally:
         ab.set_option(ab.OPT_ALL_STREAM_CHAINS, -1)
-    assert cs.count_mismatch(expected(case, src), got) == 0
+    assert cs.matches_upstream(case, src, got)
 
 
 # ---- pipelined host call: row bands over copy-in / compute / copy-out streams ----------------
@@ -162,8 +156,7 @@ def test_banded_host_call_matches_single_band(case, bands):
     finally:
         ab.set_option(ab.OPT_HOST_BANDS, -1)
     assert cs.count_mismatch(one, many) == 0
-    if o.have_ref():
-        assert cs.count_mismatch(expected(case, src), many) == 0
+    assert cs.matches_upstream(case, src, many)
 
 
 def test_banded_host_call_in_place():
@@ -209,28 +202,23 @@ FULL = [
 ]
 
 
-@needs_ref
 @pytest.mark.parametrize("name,case", FULL, ids=[f[0] for f in FULL])
 def test_full_size_baseline_configs_bit_exact(name, case):
     """BASELINE.json configs at full size, device-resident path, vs multi-threaded upstream."""
     fp, sw, sh, nw, nh, ch, ti, to, rb, kw = case
     src = o.lcg_image(sh, sw, ch, ti, seed=12345)
-    ref = o.ref_resize(src, nw, nh, to, fpclass=fp, resbits=rb, nthreads=_oracle_threads(),
-                       **cs.ref_kwargs(kw))
     got = _device_run(case, src)
-    assert cs.count_mismatch(ref, got) == 0
+    assert cs.digest(got) == _upstream_mt(case, src)
 
 
-@needs_ref
 def test_full_size_cfg4_bit_exact():
     """BASELINE configs[3] at full size, 16384^2 -> 4096^2 RGBA u16, against multi-threaded
     upstream (a few seconds per thread-second of a 1.07 GB intermediate)."""
     case = (1, 16384, 16384, 4096, 4096, 4, np.uint16, np.uint16, 16, {})
     fp, sw, sh, nw, nh, ch, ti, to, rb, kw = case
     src = o.lcg_image(sh, sw, ch, ti, seed=4)
-    ref = o.ref_resize(src, nw, nh, to, fpclass=fp, resbits=rb, nthreads=_oracle_threads())
     got = _device_run(case, src)
-    assert cs.count_mismatch(ref, got) == 0
+    assert cs.digest(got) == _upstream_mt(case, src)
 
 
 @pytest.mark.parametrize("variant", [0, 1, 2])
@@ -252,7 +240,7 @@ def test_stream_scheduling_variants_bit_exact(case, variant):
     finally:
         ab.set_option(ab.OPT_STREAM_VARIANT_H, -1)
         ab.set_option(ab.OPT_STREAM_VARIANT_V, -1)
-    assert cs.count_mismatch(expected(case, src), got) == 0
+    assert cs.matches_upstream(case, src, got)
 
 
 def test_batch_entry_matches_single_calls():
@@ -280,8 +268,7 @@ def test_batch_entry_matches_single_calls():
     lib.avirb200_plan_destroy(plan)
     rs.free_descriptor(h)
     for i in range(n):
-        want = expected(case, srcs[i].cpu().numpy())
-        assert cs.count_mismatch(want, dsts[i].cpu().numpy()) == 0, i
+        assert cs.matches_upstream(case, srcs[i].cpu().numpy(), dsts[i].cpu().numpy()), i
 
 
 def test_full_size_properties_cfg4():
@@ -320,14 +307,12 @@ def test_full_size_properties_cfg4():
     assert cs.count_mismatch(whole, d_dst.cpu().numpy()) == 0
 
 
-@needs_ref
 @pytest.mark.parametrize("nranks", [2, 5, 8])
 def test_sharded_local_matches_unsharded(nranks):
     import torch
     case = (2, 640, 720, 320, 360, 4, np.float32, np.float32, 16, {})
     fp, sw, sh, nw, nh, ch, ti, to, rb, kw = case
     src = cs.make_input(case, seed=21)
-    ref = cs.ref_output(case, src)
     rs, v = cs.resizer_and_vars(case)
     h, dp, _ = rs.descriptor(src.shape, ti, nw, nh, to, 0.0, v)
     lib = ab.lib()
@@ -348,7 +333,7 @@ def test_sharded_local_matches_unsharded(nranks):
     torch.cuda.synchronize()
     lib.avirb200_plan_destroy(plan)
     rs.free_descriptor(h)
-    assert cs.count_mismatch(ref, d_dst.cpu().numpy()) == 0
+    assert cs.matches_upstream(case, src, d_dst.cpu().numpy())
 
 
 # The fused halo exchange (AVIRB200_OPT_OVERLAP_HALO = 3: the row kernel stores the neighbours' rows into
@@ -445,18 +430,21 @@ LANCIR = [
 ]
 
 
+def _lancir_upstream(src, nw, nh, to, kw):
+    def run():
+        r, ref = o.lancir_ref(src, nw, nh, to, **kw)
+        assert r == nh
+        return ref
+    return cs.upstream(cs.lancir_key(src, nw, nh, to, kw), run)
+
+
 @pytest.mark.parametrize("sw,sh,nw,nh,ti,to,kw", LANCIR)
 def test_lancir_bit_exact(sw, sh, nw, nh, ti, to, kw):
     kw = dict(kw)
     src = o.lcg_image(sh, sw, kw.pop("C", 4), ti, seed=3)
-    if o.have_ref():
-        r, ref = o.lancir_ref(src, nw, nh, to, **kw)
-        assert r == nh
-    else:
-        pytest.skip("needs oracle/_ref")
     r, got = ab.CLancIR().resizeImage(src, nw, nh, ab.CLancIRParams(**kw), out_dtype=to)
     assert r == nh
-    assert cs.count_mismatch(ref, got) == 0
+    assert cs.digest(got) == _lancir_upstream(src, nw, nh, to, kw)
 
 
 def test_lancir_golden_fixtures():
@@ -482,7 +470,7 @@ def test_lancir_golden_fixtures():
 def test_float_source_with_input_gamma_4ch(case, kernel_path):
     src = cs.make_input(case, seed=41)
     got = cs.gpu_output(case, src)
-    assert cs.count_mismatch(expected(case, src), got) == 0
+    assert cs.matches_upstream(case, src, got)
 
 
 # ---- seeded random sweep over the whole call surface (same generator as the oracle's own) ------
@@ -523,10 +511,9 @@ def test_fuzz_product_matches_oracle(seed):
         case = (fp, sw, sh, nw, nh, ch, ti, to, rb, kw)
         src = cs.make_input(case, seed=1000 * seed + it)
         got = cs.gpu_output(case, src)
-        assert cs.count_mismatch(expected(case, src), got) == 0, cs.case_id(case)
+        assert cs.matches_upstream(case, src, got), cs.case_id(case)
 
 
-@needs_ref
 def test_lancir_fuzz_product_matches_oracle():
     """Seeded random sweep of CLancIR on the GPU: 1..4 channels, la = 2 .. 5, both scaling
     directions, offsets, explicit steps, every u8 / u16 / float type pair, against upstream."""
@@ -543,8 +530,6 @@ def test_lancir_fuzz_product_matches_oracle():
         if rng.random() < 0.3:
             kw["ox"], kw["oy"] = float(rng.uniform(-1, 1)), float(rng.uniform(-1, 1))
         src = o.lcg_image(sh, sw, ch, ti, seed=900 + it)
-        r, ref = o.lancir_ref(src, nw, nh, to, **kw)
-        assert r == nh
         r, got = ab.CLancIR().resizeImage(src, nw, nh, ab.CLancIRParams(**kw), out_dtype=to)
         assert r == nh
-        assert cs.count_mismatch(ref, got) == 0, (sw, sh, nw, nh, ch, ti, to, kw)
+        assert cs.digest(got) == _lancir_upstream(src, nw, nh, to, kw), (sw, sh, nw, nh, ch, ti, to, kw)

@@ -8,8 +8,8 @@ centring, frtest.cpp:109-111) and back, and accumulates per frequency
     PE = 20 log10 max |src*p1g - back*p2g|
 over the k sweep (frtest.cpp:224-250).  Here: same statistics, IS_UPS = 1 (upsizing first, as
 upstream's default build), fewer frequencies and a narrower image so the test runs in
-seconds.  The product must reproduce the oracle's numbers within 0.01 dB (it is bit-exact, so
-the difference is 0).
+seconds.  The product must reproduce the oracle's numbers (stored in tests/golden/upstream.json)
+within 0.01 dB (it is bit-exact, so the difference is 0).
 """
 import math
 
@@ -17,6 +17,7 @@ import numpy as np
 import pytest
 
 import avir_b200 as ab
+import cases as cs
 import oracle_ref as o
 
 pytestmark = pytest.mark.gpu
@@ -60,7 +61,6 @@ def _stats(resize, th):
     return (10.0 * math.log10(avgd / n), 10.0 * math.log10(avgd2 / n), 20.0 * math.log10(peakd), n)
 
 
-@pytest.mark.skipif(not o.have_ref(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("frac", [0.02, 0.2, 0.6, 0.95])
 def test_frtest_round_trip_statistics_match_upstream(frac):
     th = math.pi * frac
@@ -73,7 +73,7 @@ def test_frtest_round_trip_statistics_match_upstream(frac):
         return o.ref_resize(img, nw, nh, np.float32, fpclass=o.FP_DEF, k=k, resbits=16)
 
     g = _stats(gpu, th)
-    r = _stats(ref, th)
+    r = cs.upstream("frtest:%r" % frac, lambda: list(_stats(ref, th)))
     assert g[3] == r[3] == 24  # 0.95^n > 0.3
     for a, b, name in zip(g[:3], r[:3], ("FR", "DR", "PE")):
         assert abs(a - b) <= 0.01, (name, a, b)
